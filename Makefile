@@ -37,7 +37,7 @@ $(ORACLE_LIB): $(ORACLE_SRCS) $(wildcard oracle/*.h)
 
 build/tests/hlif_test: tests/cpp/hlif_test.cu $(LIB) $(HDRS)
 	@mkdir -p build/tests
-	$(NVCC) $(ARCH) -std=c++17 -O2 -Iinclude $< -o $@ -Lnvcomp_b200/lib -lnvcomp -Xlinker -rpath=$(CURDIR)/nvcomp_b200/lib
+	$(NVCC) $(ARCH) -std=c++17 -O2 -Iinclude $< -o $@ -Lnvcomp_b200/lib -lnvcomp -Xlinker -rpath='$$ORIGIN/../../nvcomp_b200/lib'
 
 clean:
 	rm -rf $(BUILD_DIR) $(LIB) $(ORACLE_LIB)

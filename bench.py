@@ -337,6 +337,27 @@ def time_decode(w: Workload, steps: int, warmup: int):
     return e0.elapsed_time(e1) / steps, [a.elapsed_time(b) for a, b in evs]
 
 
+DUMP_SAMPLE_CHUNKS = 200     # 200 x 64 KB as float32 = 52 MB, inside the 64 MB a dump may take
+
+
+def dump_outputs(w: Workload, out_dir: str):
+    """What a caller of nvcompBatched<Fmt>DecompressAsync received in the last timed step, as .npy (float32 /
+    float64) so two builds can be compared output for output: every chunk's status and decompressed size, and the
+    decompressed bytes of a fixed, seeded sample of the chunks (all of them when the batch is small enough)."""
+    import torch
+    torch.cuda.synchronize()
+    k = min(w.n, DUMP_SAMPLE_CHUNKS)
+    idx = np.sort(np.random.default_rng(0).choice(w.n, size=k, replace=False))
+    slab = w.out.slab[: w.n * CHUNK].view(w.n, CHUNK)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"statuses": w.status.cpu().numpy().astype(np.float32),
+              "decompressed_sizes": w.actual.cpu().numpy().astype(np.float64),
+              "sample_chunk_index": idx.astype(np.float64),
+              "sample_chunks": slab[torch.from_numpy(idx).to(slab.device)].cpu().numpy().astype(np.float32)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def rate_line(w: Workload, ms: float, peak: float):
     return {"chunks": w.n, "ratio": round(w.total / w.comp_total, 3), "GBps": round(w.total / ms / 1e6, 1),
             "ms": round(ms, 4), "roofline_frac": round(w.alg_bytes() / ms / 1e6 / peak, 4)}
@@ -602,6 +623,8 @@ def run_gpu(args):
     sampler = ClockSampler(torch.cuda.current_device()) if rank == 0 else None
     m = measure(kind, dataset, n, rank, world, args, sampler)
     w = m["w"]
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(w, args.dump_outputs)
     if rank == 0:
         # the timed region lasts only tens of ms; keep the identical load running (untimed) until the
         # sampler has seen ~0.6 s of it, so the clock record describes this kernel under load
@@ -885,7 +908,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip per_dataset / foreign_streams (kernel iteration)")
     ap.add_argument("--cfg5", action="store_true", help="also run BASELINE configs[4] (80,000 LZ4 chunks) at N = 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step decompressed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:
